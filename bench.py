@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W                       # B200 arm, BASELINE.json configs[1] (the headline)
   python bench.py --config {kl488,fsq488,v11long,kl41616} [--precision {bf16,exact,mixed,fma}]
   python bench.py --impl reference [--config ...] --steps K ...        # reference arm: the reference's CPU path (oracle port)
+  python bench.py ... --dump-outputs DIR                               # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of clips per GPU (weak scaling; one process per GPU under torchrun for
 N > 1).  `value` is timed with CUDA events with the inputs already resident in HBM; `e2e` goes through the public Python API
@@ -18,12 +19,15 @@ configs (BASELINE.json `configs`, SURVEY.md section 8d):
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import math
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -95,6 +99,33 @@ def load_peaks():
     return {"tflops": 1400.0, "hbm_gbs": 6650.0, "source": "fallback (B200_PROFILING.md: ~1.4 PFLOP/s sustained)"}
 
 
+DUMP_BYTES = 60 << 20    # array data of all of --dump-outputs together: the files, headers included, stay under 64 MB
+DUMP_SAMPLE_SEED = 0
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes what one step returned to the caller as out_dir/<name>.npy in float32, so that two builds can be compared
+    output for output.  Arrays go smallest first, each with an equal share of the DUMP_BYTES not yet used by the ones before
+    it.  An array larger than its share is written as <name>_sample.npy: the flattened array at sorted positions drawn
+    uniformly (with replacement) from a CPU generator seeded with DUMP_SAMPLE_SEED, as many as the share holds.  The
+    positions depend only on the element count, so the same workload gives the same sample."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    written = {}
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel())):
+        t = t.detach().float()
+        share = left // (len(arrays) - i)
+        if 4 * t.numel() > share:
+            pos = torch.randint(t.numel(), (share // 4,), generator=torch.Generator().manual_seed(DUMP_SAMPLE_SEED)).sort().values
+            t, name = t.flatten()[pos.to(t.device)], name + "_sample"
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
+        written[name] = list(a.shape)
+    return written
+
+
 # --------------------------------------------------------------------------------------------------
 # clocks
 # --------------------------------------------------------------------------------------------------
@@ -112,6 +143,8 @@ class ClockSampler:
                                           "-lms", "100"], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
         except Exception:
             self.proc = None
+        else:
+            atexit.register(self.proc.kill)   # a run that fails before stop() must not leave nvidia-smi polling
 
     def stop(self):
         if self.proc is None:
@@ -242,9 +275,25 @@ def run_reference_arm(args, c):
 # --------------------------------------------------------------------------------------------------
 # B200 arm
 # --------------------------------------------------------------------------------------------------
+def native_library():
+    """The CUDA library as the current sources build it.  That is the one build() left in the tree while it is at least as
+    new as every source and header; otherwise the sources are compiled into a temporary directory, removed at exit, and that
+    build is loaded.  So the timed kernels always match the sources, and nothing is written into the tree, which may be
+    read-only."""
+    from vidtok_b200 import _native as N
+    from vidtok_b200 import build as vb
+    if vb.is_stale():
+        tmp = tempfile.mkdtemp(prefix="vidtok_b200_")
+        atexit.register(shutil.rmtree, tmp, True)
+        print(f"bench.py: {vb.LIB} is missing or older than its sources; building them in {tmp}", file=sys.stderr, flush=True)
+        N.LIB_PATH = vb.build(force=True, out_dir=tmp)
+    lib = N.lib()
+    assert lib.vt_abi_version() == 2
+    return lib
+
+
 def run_b200_arm(args, c):
-    import __graft_entry__ as ge
-    ge.build()
+    native_library()   # before anything loads the library
     from vidtok_b200 import _native as N
     from vidtok_b200 import dist as vdist
     from vidtok_b200.compat_util import instantiate_from_config
@@ -356,6 +405,9 @@ def run_b200_arm(args, c):
     ms = float(vdist.allreduce_max(ms)[0])
     frames = world * B * T * args.steps
     value = frames / (ms / 1e3)
+    dumped = None
+    if args.dump_outputs and rank == 0:   # what the last timed step returned (z, dec, reg_log), copied after the timed region
+        dumped = dump_outputs(args.dump_outputs, {"z": z, "dec": dec, **log})
 
     # ---- end to end through the public API with host buffers
     run_e2e(2)
@@ -490,6 +542,8 @@ def run_b200_arm(args, c):
             "psnr": parity,
             "parity": parity,   # same record under the name VERDICT r1 asked for (PSNR delta; FSQ code mismatches for fsq488)
         }
+        if dumped is not None:
+            line["dumped_outputs"] = {"dir": args.dump_outputs, "shapes": dumped, "sample_seed": DUMP_SAMPLE_SEED}
         print(json.dumps(line), flush=True)
     if torch.distributed.is_initialized():
         torch.distributed.destroy_process_group()
@@ -505,7 +559,13 @@ def main():
     ap.add_argument("--precision", default=None, choices=["bf16", "exact", "mixed", "fma"], help="default: the config's")
     ap.add_argument("--batch", type=int, default=0, help="clips per GPU (default: the config's)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32, at most 64 MB; B200 arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the B200 arm's outputs")
     c = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference_arm(args, c)   # CPU only: the CUDA library is neither built nor loaded here

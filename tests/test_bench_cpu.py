@@ -48,6 +48,45 @@ def test_importing_bench_does_not_load_the_cuda_library():
     assert out.stdout.strip().endswith("False")
 
 
+def test_dump_outputs_fit_the_budget_in_float32_and_sample_reproducibly(tmp_path):
+    import numpy as np
+    g = torch.Generator().manual_seed(0)
+    outs = {"z": torch.randn(8, 4, 5, 32, 32, generator=g).bfloat16(), "dec": torch.randn(8, 3, 17, 256, 256, generator=g),
+            "kl_loss": torch.tensor(2.5), "indices": torch.randint(0, 32768, (8, 5, 32, 32), generator=g, dtype=torch.int32)}
+    shapes = bench.dump_outputs(str(tmp_path / "a"), outs)
+    assert set(shapes) == {"z", "kl_loss", "indices", "dec_sample"}
+    assert shapes["z"] == [8, 4, 5, 32, 32] and shapes["kl_loss"] == [] and shapes["indices"] == [8, 5, 32, 32]
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64e6
+    a = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert all(v.dtype == np.float32 for v in a.values())
+    assert np.array_equal(a["z"], outs["z"].float().numpy()) and float(a["kl_loss"]) == 2.5
+    assert np.array_equal(a["indices"], outs["indices"].numpy().astype(np.float32))
+    assert np.isin(a["dec_sample"][:1000], outs["dec"].numpy()).all()
+    bench.dump_outputs(str(tmp_path / "b"), outs)
+    assert np.array_equal(np.load(tmp_path / "b" / "dec_sample.npy"), a["dec_sample"])
+    # two arrays over the budget share it: neither sample is empty
+    shapes = bench.dump_outputs(str(tmp_path / "c"), {"a": torch.zeros(20_000_000), "b": torch.zeros(30_000_000)})
+    assert shapes == {"a_sample": [bench.DUMP_BYTES // 8], "b_sample": [bench.DUMP_BYTES // 8]}
+
+
+def test_stale_library_is_rebuilt_outside_the_tree():
+    """bench.py never times a library older than its sources, and never writes into the tree: a stale (here: missing)
+    in-tree library makes it compile the current sources into a temporary directory and load that."""
+    import subprocess
+    from vidtok_b200 import build as vb
+    before = {p: os.path.getmtime(p) for p in (vb.LIB, vb.OBJ)}
+    code = ("import sys; sys.path.insert(0, %r); import bench; from vidtok_b200 import build as vb, _native as N; "
+            "vb.LIB = vb.LIB + '.missing'; assert vb.is_stale(); bench.native_library(); print(N.LIB_PATH)" % ROOT)
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=1200)
+    assert r.returncode == 0, r.stderr[-3000:]
+    built = r.stdout.strip().splitlines()[-1]
+    assert not built.startswith(ROOT) and "older than its sources" in r.stderr
+    assert not os.path.exists(built)   # the temporary build is removed at exit
+    assert before == {p: os.path.getmtime(p) for p in (vb.LIB, vb.OBJ)} and not os.path.exists(vb.LIB + ".missing")
+    assert not vb.is_stale()
+
+
 def test_cpu_sample_scaling_is_in_full_size_frames():
     c = bench.CONFIGS["kl488"]
     assert bench.cpu_units_scale(c, 17, 256) == pytest.approx(17.0)

@@ -2,13 +2,20 @@
 scripts import unchanged -- hot-path modules resolve to the B200 shims, everything else (vidtok.data.*, vidtok.modules.lpips)
 to the reference -- and `load_model_from_config` (scripts/inference_evaluate.py:26-32) builds the B200 engine.
 
-Needs the reference checkout (VIDTOK_REFERENCE_ROOT or /root/reference): skipped on the GPU box.  Runs in subprocesses so
-the import state of the test process is untouched.  Also: the oracle pin is reproducible (oracle/make_golden.py), the
-oracle's parameter table equals the reference's state_dict, and compute_ssim equals the reference formula."""
+The reference checkout is the one oracle/ref_shim.py locates (VIDTOK_REFERENCE_ROOT overrides it), the same one the golden
+fixtures were made from.  Without one, the checks run against a stand-in checkout with the reference's package layout,
+and the configs come from tests/golden/zoo_manifest.json.gz (the `model:` sections of the reference's YAMLs): where the
+overlay resolves each module, which engine the config builds, and its parameter count.  What only the reference's own
+scripts can show -- that they import unchanged, that their compute_ssim is ours and that their dataset derives from the
+checkout's vidtok.data.vidtok -- is checked with the reference only.  Runs in subprocesses so the import state of the
+test process is untouched.  Also: the oracle pin is reproducible (oracle/make_golden.py, needs the reference), the oracle's
+parameter table equals the reference's state_dict, and compute_ssim equals the reference formula."""
+import gzip
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import textwrap
 
 import numpy as np
@@ -17,9 +24,31 @@ import torch
 import torch.nn.functional as F
 
 from conftest import GOLDEN_DIR, ROOT, golden_cases, load_golden
+from oracle import ref_shim
 
-REF = os.environ.get("VIDTOK_REFERENCE_ROOT", "/root/reference")
-needs_ref = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "vidtok", "modules")), reason="reference checkout not present")
+REF = ref_shim.REFERENCE_ROOT
+HAVE_REF = ref_shim.reference_available()
+needs_ref = pytest.mark.skipif(not HAVE_REF, reason="reference checkout not present")
+ZOO = json.load(gzip.open(os.path.join(GOLDEN_DIR, "zoo_manifest.json.gz"), "rt"))
+
+# The part of the reference's layout that the inference scripts import from and vidtok/__init__.py looks for: `vidtok` is a
+# namespace package (no __init__.py) holding data/ and modules/util.py.
+STANDIN = {
+    "vidtok/data/vidtok.py": "class VidTokValDataset:\n    pass\n",
+    "vidtok/modules/util.py": "",
+    "vidtok/modules/lpips.py": "class LPIPS:\n    pass\n",
+}
+
+
+@pytest.fixture
+def checkout(tmp_path):
+    if HAVE_REF:
+        return REF
+    for rel, text in STANDIN.items():
+        (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+        (tmp_path / rel).write_text(text)
+    return str(tmp_path)
+
 
 # Modules the scripts import that are absent offline (SURVEY.md section 0.5).  Stubs only: no behaviour is borrowed.
 STUBS = textwrap.dedent('''
@@ -54,53 +83,70 @@ STUBS = textwrap.dedent('''
 ''')
 
 
-def run_py(code, extra_env=None):
+def run_py(checkout, *parts):
+    """Runs the code `parts` (each dedented) in a fresh interpreter with this repo, then `checkout`, on PYTHONPATH."""
     env = dict(os.environ)
-    env["PYTHONPATH"] = os.pathsep.join([ROOT, REF])   # INTEGRATION.md: this repo first, then the reference checkout
-    env.update(extra_env or {})
-    r = subprocess.run([sys.executable, "-c", STUBS + textwrap.dedent(code)], capture_output=True, text=True, env=env, cwd="/tmp",
+    env["PYTHONPATH"] = os.pathsep.join([ROOT, checkout])   # INTEGRATION.md: this repo first, then the reference checkout
+    code = "".join(textwrap.dedent(p) for p in ((STUBS,) if HAVE_REF else ()) + parts)
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd=tempfile.gettempdir(),
                        timeout=600)
     assert r.returncode == 0, r.stdout + "\n" + r.stderr
     return r.stdout
 
 
-@needs_ref
-def test_reference_scripts_import_unchanged_and_build_the_b200_engine():
-    cfg = os.path.join(REF, "configs", "vidtok_kl_causal_488_4chn.yaml")
-    out = run_py(f'''
+def load_model_code(config):
+    """Code that builds `model` from the reference config `config` (a path under configs/) as scripts/inference_evaluate.py
+    does, and names the script, its compute_ssim and the base class of its dataset (all None with the stand-in).  With the reference:
+    its own script, unmodified, on the YAML.  With the stand-in: the script's imports (:20-23) and the steps of its
+    load_model_from_config (:26-32) on the recorded `model:` section."""
+    if HAVE_REF:
+        return f"""
+            import inspect
+            import scripts.inference_evaluate as ev          # the reference's script, unmodified
+            import scripts.inference_reconstruct as rc
+            model = ev.load_model_from_config({os.path.join(REF, "configs", config)!r}, None)
+            script, ssim_fn, dataset_cls = inspect.getfile(ev), ev.compute_ssim, ev.MultiVideoDataset.__mro__[1].__module__
+        """
+    return f"""
+        from vidtok.data.vidtok import VidTokValDataset
+        from vidtok.modules.lpips import LPIPS
+        from vidtok.modules.util import compute_psnr, compute_ssim, instantiate_from_config, print0
+        cfg = {ZOO[config]["model"]!r}
+        cfg["params"].update(ckpt_path=None, ignore_keys=[], verbose=False)
+        model = instantiate_from_config(cfg)
+        script = ssim_fn = dataset_cls = None
+    """
+
+
+def test_reference_scripts_import_unchanged_and_build_the_b200_engine(checkout):
+    out = run_py(checkout, load_model_code("vidtok_kl_causal_488_4chn.yaml"), '''
         import inspect, json
-        import scripts.inference_evaluate as ev          # the reference's script, unmodified
-        import scripts.inference_reconstruct as rc
         import vidtok, vidtok.data.vidtok, vidtok.modules.lpips, vidtok.modules.util, vidtok.models.autoencoder
-        model = ev.load_model_from_config({cfg!r}, None)
-        print(json.dumps({{
-            "script": inspect.getfile(ev), "dataset": inspect.getfile(vidtok.data.vidtok), "lpips": inspect.getfile(vidtok.modules.lpips),
+        print(json.dumps({
+            "script": script, "dataset": inspect.getfile(vidtok.data.vidtok), "lpips": inspect.getfile(vidtok.modules.lpips),
+            "util": inspect.getfile(vidtok.modules.util),
             "engine": inspect.getfile(type(model)), "engine_cls": type(model).__name__, "is_causal": model.is_causal,
             "tdf": model.encoder.time_downsample_factor, "has_tiling": hasattr(model, "use_tiling"),
-            "ssim": ev.compute_ssim is vidtok.modules.util.compute_ssim, "nparams": len(model.state_dict()),
-            "dataset_cls": ev.MultiVideoDataset.__mro__[1].__module__,
-        }}))
+            "ssim": ssim_fn is vidtok.modules.util.compute_ssim, "nparams": len(model.state_dict()), "dataset_cls": dataset_cls,
+        }))
     ''')
     info = json.loads(out.strip().splitlines()[-1])
-    assert info["script"].startswith(REF) and info["dataset"].startswith(REF) and info["lpips"].startswith(REF)
+    if HAVE_REF:
+        assert info["script"].startswith(REF) and info["ssim"] is True and info["dataset_cls"] == "vidtok.data.vidtok"
+    assert info["dataset"].startswith(checkout) and info["lpips"].startswith(checkout) and info["util"].startswith(ROOT)
     assert info["engine"].startswith(ROOT) and info["engine_cls"] == "AutoencodingEngine"
-    assert info["is_causal"] is True and info["tdf"] == 4 and info["has_tiling"] is False and info["ssim"] is True
-    assert info["nparams"] == 416 and info["dataset_cls"] == "vidtok.data.vidtok"
+    assert info["is_causal"] is True and info["tdf"] == 4 and info["has_tiling"] is False and info["nparams"] == 416
 
 
-@needs_ref
-def test_v11_config_resolves_to_the_tiling_engine():
-    cfg = os.path.join(REF, "configs", "vidtok_v1_1", "vidtok_kl_causal_488_16chn_v1_1.yaml")
-    out = run_py(f'''
+def test_v11_config_resolves_to_the_tiling_engine(checkout):
+    out = run_py(checkout, load_model_code("vidtok_v1_1/vidtok_kl_causal_488_16chn_v1_1.yaml"), '''
         import json
-        import scripts.inference_evaluate as ev
-        model = ev.load_model_from_config({cfg!r}, None)
         # scripts/inference_evaluate.py:144-150
         assert hasattr(model, "use_tiling")
         model.use_tiling = True; model.t_chunk_enc = 16
         model.t_chunk_dec = model.t_chunk_enc // model.encoder.time_downsample_factor; model.use_overlap = True
-        print(json.dumps({{"cls": type(model).__name__, "z": model.spec.z_channels, "interp": model.spec.interpolation_mode,
-                           "chunks": model.build_chunk_start_end(129)[:3]}}))
+        print(json.dumps({"cls": type(model).__name__, "z": model.spec.z_channels, "interp": model.spec.interpolation_mode,
+                          "chunks": model.build_chunk_start_end(129)[:3]}))
     ''')
     info = json.loads(out.strip().splitlines()[-1])
     assert info == {"cls": "AutoencodingEngineV11", "z": 16, "interp": "trilinear", "chunks": [[0, 1], [1, 17], [17, 33]]}
